@@ -2,7 +2,7 @@
 """bench.py -- trajectories/sec of the dopri5 hot path on BASELINE.json's configs[1]
 (dopri5 adaptive, batch=65536 dim=128 linear ODE y' = A y, float32, rtol=1e-5, atol=1e-7, t in [0, 10]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one complete odeint solve of the batch (about 74 step attempts, 446 func evaluations).
 N > 1 (torchrun, one rank per GPU): every rank integrates its own 65536 trajectories (weak scaling,
@@ -19,6 +19,10 @@ public API with pinned HOST buffers (H2D of y0 and D2H of y(t_end) inside the ti
 `roofline` is the dominant kernel group's algorithmic bytes / its CUDA-event time against the measured
 HBM peak; `cpu_baseline` is the unmodified reference (baseline/_ref; the CPU oracle only if it did not travel) on a bounded
 sample.  --impl reference times that CPU implementation alone on the host cores.
+
+--dump-outputs DIR writes the solution the last timed step returned as DIR/solution.npy (float32, the rows of a
+fixed seeded sample of the trajectories, see dump_outputs), so that two builds can be compared output for output:
+the inputs are the same in every run with the same arguments.
 """
 import argparse
 import ctypes as C
@@ -128,6 +132,7 @@ TRAFFIC_FUSED = {"bytes": 946.1e6, "source": "static: dram__bytes_read+write of 
 TRAFFIC_ATTEMPT = {"bytes": 82.8e6, "source": "static: dram__bytes_read.sum 67.4 MB (= y0 + k_0, the algorithmic reads) + dram__bytes_write.sum "
                                                   "15.4 MB of one k_linear_attempt launch, ncu --set full (profiles/r2_ncu_full_k_linear_attempt_raw.csv): "
                                                   "most of the 67 MB of candidates it writes is still in L2 when the launch ends; not measured by this run"}
+DUMP_ROWS = 32768          # trajectories kept by --dump-outputs: [len(t), 32768, 128] float32 = 33.5 MB
 FULL_ATTEMPTS = 74         # step attempts of the full workload (reference, oracle and CUDA path agree; SURVEY.md section 6)
 CPU_SAMPLE_T_END = 1.0     # the CPU sample integrates the FULL batch over t in [0, 1] (9 of the 74 attempts, + the start-up work)
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")      # the unmodified reference, `pip install --target` (DESIGN.md section 7)
@@ -168,9 +173,19 @@ class _Rec(torch.nn.Module):
         self.n_reject += 1
 
 
+def dump_outputs(path, solution):
+    """Writes the solution [len(t), batch, DIM] as path/solution.npy in float32: the rows of DUMP_ROWS trajectories
+    drawn once from a generator with a fixed seed (in ascending order), the same rows in every run."""
+    import numpy as np
+    n = solution.shape[1]
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:min(n, DUMP_ROWS)].sort().values
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "solution.npy"), solution.detach().cpu()[:, rows].to(torch.float32).numpy())
+
+
 def cpu_run(batch, threads, t_end=T_SPAN[1]):
     """One solve of the workload at `batch` rows over t in [0, t_end] on the host cores: the unmodified reference
-    when available (kind 'reference'), else the CPU oracle (kind 'port').  Returns (seconds, attempts, kind)."""
+    when available (kind 'reference'), else the CPU oracle (kind 'port').  Returns (seconds, attempts, kind, solution)."""
     torch.set_num_threads(threads)
     f, y0, _, _ = make_problem("cpu", batch)
     t = torch.tensor([T_SPAN[0], t_end])
@@ -179,27 +194,27 @@ def cpu_run(batch, threads, t_end=T_SPAN[1]):
         if ref is not None:
             rec = _Rec(f)
             t0 = time.perf_counter()
-            ref.odeint(rec, y0, t, method="dopri5", rtol=RTOL, atol=ATOL)
+            sol = ref.odeint(rec, y0, t, method="dopri5", rtol=RTOL, atol=ATOL)
             dt = time.perf_counter() - t0
-            return dt, rec.n_accept + rec.n_reject, "reference"
+            return dt, rec.n_accept + rec.n_reject, "reference", sol
         from oracle import ode_oracle as O
         r = {}
         t0 = time.perf_counter()
-        O.odeint_adaptive(f, y0, t, "dopri5", rtol=RTOL, atol=ATOL, record=r)
+        sol = O.odeint_adaptive(f, y0, t, "dopri5", rtol=RTOL, atol=ATOL, record=r)
         dt = time.perf_counter() - t0
-        return dt, r["n_accept"] + r["n_reject"], "port"
+        return dt, r["n_accept"] + r["n_reject"], "port", sol
 
 
 def cpu_sample(threads):
     """Bounded CPU sample of the workload: all 65536 rows (so the arrays are as cache-unfriendly as in the real
     job -- a smaller batch fits the host's L3 and runs up to 10x faster per row), but only the first part of the
     time span; the per-attempt cost is constant, so a sample that completes a/74 of every trajectory's attempts in
-    s seconds runs at B*(a/74)/s trajectories per second."""
-    secs, attempts, kind = cpu_run(B_PER_GPU, threads, CPU_SAMPLE_T_END)
+    s seconds runs at B*(a/74)/s trajectories per second.  Also returns the sample's solution."""
+    secs, attempts, kind, sol = cpu_run(B_PER_GPU, threads, CPU_SAMPLE_T_END)
     value = B_PER_GPU * (attempts / FULL_ATTEMPTS) / secs
     desc = ("all %d rows, t in [0,%g]: %d of the %d step attempts per sample, %.2f s per sample; "
             "value = rows x (attempts/74) / seconds" % (B_PER_GPU, CPU_SAMPLE_T_END, attempts, FULL_ATTEMPTS, secs))
-    return value, secs, desc, kind
+    return value, secs, desc, kind, sol
 
 
 def run_reference(args):
@@ -213,12 +228,14 @@ def run_reference(args):
     warm = max(1, min(args.warmup, 2))            # the CPU path has no lazy initialisation beyond its first call
     for _ in range(warm):
         cpu_sample(threads)
-    steps = max(1, args.steps)
+    steps = args.steps
     vals, secs = [], []
     for _ in range(steps):
-        v, s_, desc, kind = cpu_sample(threads)
+        v, s_, desc, kind, sol = cpu_sample(threads)
         vals.append(v)
         secs.append(s_)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sol)
     value = sum(vals) / len(vals)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "trajectories/s", "n_gpus": args.gpus,
@@ -376,6 +393,8 @@ def run_ours(args):
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     launches = stats.get("launches", 0) - launches0
     clocks = sampler.stop() if rank == 0 else None
     # ---- end to end: pinned host y0 -> device -> solve -> y(t_end) back to pinned host -----------------
@@ -443,7 +462,7 @@ def run_ours(args):
         achieved = comb_bytes / (comb_ms * 1e-3) / 1e9
         group = (comb_bytes + norm_bytes) / (group_ms * 1e-3) / 1e9
         threads = cpu_threads()
-        cpu_val, _cpu_s, cpu_desc, cpu_kind = cpu_sample(threads) if args.cpu_baseline and world == 1 else (None,) * 4
+        cpu_val, _cpu_s, cpu_desc, cpu_kind, _ = cpu_sample(threads) if args.cpu_baseline and world == 1 else (None,) * 5
         total_traj = rows * world * args.steps
         line = {
             "metric": METRIC, "value": total_traj / (ms * 1e-3), "unit": "trajectories/s", "n_gpus": world,
@@ -553,13 +572,22 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def positive_int(v):
+    n = int(v)
+    if n < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %s" % v)
+    return n
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps (one complete solve each)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution of the last one as DIR/solution.npy (rank 0's rows)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="N > 1: weak = 65536 trajectories per rank (configs[4]); strong = 65536 split over the ranks")
     ap.add_argument("--generic", action="store_true",

@@ -18,6 +18,8 @@ Outputs (committed):
     adjoint_many.pt       odeint_adjoint on a field with 80 parameter tensors (default norm: 83 segments)
     adams.json, adams.pt  Adams-Bashforth(-Moulton) weight tables and explicit_adams / implicit_adams solutions, events
     backprop.pt           gradients of plain odeint (autograd through the reference's solver operations)
+    seam_objects.json     identities of the objects the reference hands a registered solver (default norm, null
+                          callback, perturb wrapper) and where its SOLVERS registry lives
 """
 import json
 import os
@@ -67,6 +69,23 @@ def dump_tableaus():
                      "c_err": tab.c_error.tolist(), "c_mid": cls.mid.tolist(), "order": cls.order, "fsal": fsal,
                      "n_stages": len(tab.alpha)}
     with open(os.path.join(HERE, "tableaus.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
+def seam_objects():
+    """What torchdiffeq_b200.plugin has to recognise in the reference's objects, by name only (misc.py:11, :18-33,
+    :174-197; odeint.py:19-46; adjoint.py:4)."""
+    import importlib
+    misc = importlib.import_module("torchdiffeq._impl.misc")
+    odeint_mod = importlib.import_module("torchdiffeq._impl.odeint")
+    ident = lambda fn: {"name": fn.__name__, "module": fn.__module__, "qualname": fn.__qualname__}
+    wrapped = misc._PerturbFunc(abs)
+    out = {"_rms_norm": ident(misc._rms_norm), "_mixed_norm": ident(misc._mixed_norm),
+           "_null_callback": ident(misc._null_callback),
+           "_PerturbFunc": {"class": type(wrapped).__name__, "base_func_attr": wrapped.base_func is abs},
+           "registry": {"module": odeint_mod.__name__, "methods": sorted(odeint_mod.SOLVERS),
+                        "shared_with_adjoint": importlib.import_module("torchdiffeq._impl.adjoint").SOLVERS is odeint_mod.SOLVERS}}
+    with open(os.path.join(HERE, "seam_objects.json"), "w") as f:
         json.dump(out, f, indent=1)
 
 
@@ -452,5 +471,6 @@ if __name__ == "__main__":
     backprop()
     adjoint_many()
     adams()
+    seam_objects()
     for fn in sorted(os.listdir(HERE)):
         print(fn, os.path.getsize(os.path.join(HERE, fn)))

@@ -1,11 +1,10 @@
-"""The registry-seam plug-in (torchdiffeq_b200/plugin.py) driven through the REFERENCE's own front end: the
-unmodified reference package (baseline/_ref, or /root/reference in the build container) keeps its odeint /
-odeint_adjoint, _check_inputs, tuple plumbing, event wrappers and adjoint; only SOLVERS[method] is replaced
-(odeint.py:19-46, :92-97; adjoint.py:4 shares the dict).  Mirrors the reference's tests/odeint_tests.py,
-api_tests.py, norm_tests.py, event_tests.py and gradient_tests.py on CUDA tensors.  When the reference is not
-importable a stand-in for the caller side of the seam (tests/seam_frontend.py) is used and the adjoint cases skip."""
+"""The registry-seam plug-in (torchdiffeq_b200/plugin.py) driven through the caller side of the reference's seam:
+the plug-in replaces only SOLVERS[method] (odeint.py:19-46, :92-97; adjoint.py:4 shares the dict) and the front end
+keeps its odeint / odeint_adjoint, _check_inputs, tuple plumbing, event wrappers and adjoint.  That front end is
+tests/seam_frontend.py, a stand-in that hands the solver exactly what the reference's does.  Mirrors the
+reference's tests/odeint_tests.py, api_tests.py, norm_tests.py, event_tests.py and gradient_tests.py on CUDA tensors,
+against the reference's CPU goldens."""
 import os
-import sys
 
 import pytest
 import torch
@@ -15,38 +14,19 @@ import problems as P
 pytestmark = pytest.mark.gpu
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 G = os.path.join(HERE, "golden")
 ld = lambda name: torch.load(os.path.join(G, name), weights_only=False)
 DEV = "cuda:0"
 
 
-def _import_reference():
-    for path in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(path, "torchdiffeq")):
-            if path not in sys.path:
-                sys.path.insert(0, path)
-            import torchdiffeq
-            return torchdiffeq
-    return None
-
-
 @pytest.fixture(scope="module")
 def front():
-    """(odeint, odeint_adjoint or None, is_reference) with the plug-in registered for the duration of the module."""
+    """(odeint, odeint_adjoint) of the seam's caller side with the plug-in registered for the duration of the module."""
+    import seam_frontend as sf
     from torchdiffeq_b200 import plugin
-    ref = _import_reference()
-    if ref is not None:
-        import importlib
-        solvers = importlib.import_module("torchdiffeq._impl.odeint").SOLVERS
-        replaced = plugin.register(solvers)
-        yield ref.odeint, ref.odeint_adjoint, True
-        plugin.unregister(replaced, solvers)
-    else:
-        import seam_frontend as sf
-        replaced = plugin.register(sf.SOLVERS)
-        yield sf.odeint, None, False
-        plugin.unregister(replaced, sf.SOLVERS)
+    replaced = plugin.register(sf.SOLVERS)
+    yield sf.odeint, sf.odeint_adjoint
+    plugin.unregister(replaced, sf.SOLVERS)
 
 
 class Counted(torch.nn.Module):
@@ -68,7 +48,7 @@ STAGES = {"dopri5": 6, "dopri8": 13, "tsit5": 6, "bosh3": 3, "fehlberg2": 2, "ad
 def test_seam_zoo(front, key):
     """tests/odeint_tests.py:17-58 through the seam: every registered method, both dtypes, both directions; the
     default is the reference's exact call sequence, so func's own NFE counter equals 2 + S*attempts."""
-    odeint, _, _ = front
+    odeint, _ = front
     ode, method, dt, direction = key.split("/")
     dtype = getattr(torch, dt)
     case = ZOO[key]
@@ -95,7 +75,7 @@ def test_seam_zoo(front, key):
 def test_seam_tuple_state_and_options(front):
     """api_tests.py:12-26 (tuple == tensor), tuple tolerances (misc.py:115-123) and the anonymous norm closure the
     seam hands over for tuple states (compatibility path), against the reference's CPU goldens."""
-    odeint, _, _ = front
+    odeint, _ = front
     case = ld("options.pt")["tuple"]
     A = P.skew_matrix(6, torch.float64).to(DEV)
 
@@ -124,7 +104,7 @@ def test_seam_tuple_state_and_options(front):
 def test_seam_custom_norm_and_callbacks(front):
     """norm_tests.py style: a user norm reaches the solver through options['norm']; callbacks arrive as attributes
     of the wrapped func (misc.py:311-332) and fire in the reference's order and number."""
-    odeint, _, _ = front
+    odeint, _ = front
     f, y0, t, _ = P.construct_problem(DEV, ode="linear", dtype=torch.float64)
     calls = {"n": 0}
 
@@ -167,7 +147,7 @@ EV = ld("events.pt")
 @pytest.mark.parametrize("key", sorted(k for k in EV if k.count("/") == 3 and k.split("/")[1] in ("dopri5", "bosh3")))
 def test_seam_events(front, key):
     """event_tests.py:14-49 through solver.integrate_until_event (odeint.py:97)."""
-    odeint, _, _ = front
+    odeint, _ = front
     ode, method, dt, direction = key.split("/")
     dtype = getattr(torch, dt)
     case = EV[key]
@@ -188,12 +168,10 @@ def test_seam_events(front, key):
 
 @pytest.mark.parametrize("key", sorted(ld("adjoint_mlp.pt")))
 def test_seam_adjoint_gradients(front, key):
-    """gradient_tests.py:34-86 style: the reference's odeint_adjoint with our solver registered -- its backward
+    """gradient_tests.py:34-86 style: odeint_adjoint with our solver registered -- its backward
     instantiates SOLVERS[method] once per output interval with the augmented flat state and an anonymous norm
     closure (adjoint.py:134-138, :247-288); gradients against the CPU reference's to 1e-4 relative."""
-    _, odeint_adjoint, is_ref = front
-    if not is_ref:
-        pytest.skip("needs the reference's odeint_adjoint front end")
+    _, odeint_adjoint = front
     case = ld("adjoint_mlp.pt")[key]
     name, norm, dt = key.split("/")
     dtype = getattr(torch, dt)
@@ -214,7 +192,7 @@ def test_seam_adjoint_gradients(front, key):
 
 def test_seam_graph_mode_opt_in(front):
     """options={'graph': True} through the seam: captured step body inside the device loop, same result."""
-    odeint, _, _ = front
+    odeint, _ = front
     f = P.BatchedLinear(128).to(DEV)
     y0 = torch.randn(512, 128, generator=torch.Generator().manual_seed(1)).to(DEV)
     t = torch.linspace(0, 2, 5).to(DEV)
@@ -228,7 +206,7 @@ def test_seam_graph_mode_opt_in(front):
 def test_seam_adams(front, method):
     """The Adams methods through the seam (odeint.py:31-42 registers AdamsBashforth / AdamsBashforthMoulton; the
     constructor receives odeint's rtol/atol, fixed_adams.py:167-175)."""
-    odeint, _, _ = front
+    odeint, _ = front
     AD = ld("adams.pt")
     for direction in ("fwd", "rev"):
         case = AD["linear/%s/float64/%s/step" % (method, direction)]
