@@ -37,7 +37,16 @@ typedef enum {
     TDQ_ERR_UNSUPPORTED = 3
 } tdq_status;
 
-typedef enum { TDQ_F32 = 0, TDQ_F64 = 1 } tdq_dtype;
+/* State dtypes.  A complex state (TDQ_C64 = complex64, TDQ_C128 = complex128) is stored as interleaved (re, im)
+ * pairs of its component dtype (float32 / float64).  For a complex code every element count `n`, every segment
+ * offset and length and every chunk-table entry counts COMPLEX elements, and every state, stage, coefficient and
+ * solution buffer holds n complex values.  Everything that is a real scalar or a real coefficient array stays in the
+ * component dtype: tdq_options.dtype, the control block (tdq_ctrl_init takes only TDQ_F32 / TDQ_F64, and tstage /
+ * taux are component-dtype scalars), the dtype passed to tdq_prepare_attempt, tdq_controller, tdq_initial_step_h0 /
+ * _finish, the dt / slope / cubic-weight arrays of the fixed-grid launchers, and the ratio of tdq_controller.
+ * Norms use the complex modulus: |z| = hypot(re, im), one tolerance per complex element, err/tol = err*fl(1/tol)
+ * componentwise, and each complex element contributes |err/tol|^2 once.  complex32 has no code. */
+typedef enum { TDQ_F32 = 0, TDQ_F64 = 1, TDQ_C64 = 2, TDQ_C128 = 3 } tdq_dtype;
 
 /* Solver status word kept in the control block (device) and mirrored into the mailbox.
  * Mirrors the three assertions of the reference's adaptive loop. */

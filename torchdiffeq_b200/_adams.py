@@ -64,9 +64,10 @@ class AdamsEngine(FixedGridEngine):
         super().__init__(fn, n, dtype, device, method="rk4", t_sign=t_sign, perturb=perturb, graph=False,
                          callbacks=callbacks, pieces=pieces, interp=interp)
         self.implicit, self.max_iters, self.max_order = bool(implicit), int(max_iters), int(max_order)
-        # fixed_adams.py:174-175: tolerances of the corrector's stopping test, in the state dtype
-        self.rtol = float(torch.as_tensor(rtol, dtype=torch.float64).to(dtype))
-        self.atol = float(torch.as_tensor(atol, dtype=torch.float64).to(dtype))
+        # fixed_adams.py:174-175: tolerances of the corrector's stopping test, in the state dtype (its real part for a
+        # complex state: the imaginary part is zero)
+        self.rtol = float(torch.as_tensor(rtol, dtype=torch.float64).to(self.rdtype))
+        self.atol = float(torch.as_tensor(atol, dtype=torch.float64).to(self.rdtype))
         self.prev_f = collections.deque(maxlen=self.max_order - 1)
         self.prev_t = None
         self.graph_opt = False
@@ -111,12 +112,13 @@ class AdamsEngine(FixedGridEngine):
         if getattr(self, "_event_step", None) is not None:                      # event stepping: explicit (t0, dt, t1)
             t0, dt, t1 = self._event_step
             dt64 = float(torch.as_tensor(dt, dtype=torch.float64)) if not torch.is_tensor(dt) else float(dt.double())
-            dt_T = float(torch.as_tensor(dt64, dtype=torch.float64).to(T)) if not torch.is_tensor(dt) else float(dt.to(T))
+            dt_T = float(torch.as_tensor(dt64, dtype=torch.float64).to(self.rdtype)) if not torch.is_tensor(dt) \
+                else float(dt.to(self.rdtype))
         else:
             k = self._step_index
             t0, t1 = self._grid_cpu[k], self._grid_cpu[k + 1]
             dtt = t1 - t0                                                        # t's dtype (solvers.py:112)
-            dt64, dt_T = float(dtt.double()), float(dtt.to(T))
+            dt64, dt_T = float(dtt.double()), float(dtt.to(self.rdtype))
             self._step_index += 1
         sgn = self.t_sign
         # func outputs of earlier steps are kept: a func that reuses one output buffer must be copied
@@ -170,6 +172,8 @@ class AdamsEngine(FixedGridEngine):
                 # fixed_adams.py:188-191: max |(|dy_old - dy|) / (atol + rtol*max(|dy_old|, |dy|))| < 1 -- a host decision
                 err = torch.abs(dy_old - dy)
                 tol = self.atol + self.rtol * torch.max(dy_old.abs(), dy.abs())
+                if T.is_complex:                     # the reference's tolerances are complex there: err/(tol + 0i)
+                    tol = tol.to(T)
                 converged = bool((err / tol).abs().max() < 1)
                 if converged:
                     break

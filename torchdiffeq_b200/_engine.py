@@ -32,7 +32,17 @@ import torch
 
 from . import _lib
 
-_DTYPES = {torch.float32: _lib.TDQ_F32, torch.float64: _lib.TDQ_F64}
+_DTYPES = {torch.float32: _lib.TDQ_F32, torch.float64: _lib.TDQ_F64,
+           torch.complex64: _lib.TDQ_C64, torch.complex128: _lib.TDQ_C128}
+
+
+def state_codes(dtype):
+    """(libtdq code of the state dtype, code of its real component dtype).  Launchers that move or combine the state
+    take the first; the control block and everything scalar (time, step size, error ratio) take the second."""
+    if dtype not in _DTYPES:
+        raise _lib.TdqError("unsupported state dtype %s (float32, float64, complex64 and complex128 are implemented)"
+                            % dtype)
+    return _DTYPES[dtype], _DTYPES[dtype.to_real()]
 
 
 def _stream():
@@ -172,14 +182,13 @@ class AdaptiveEngine:
                  agree_fn=None, exchange=None, callbacks=None, keep_interp=False, device_loop="auto", post_fn=None):
         if device.type != "cuda":
             raise _lib.TdqError("torchdiffeq_b200 runs on CUDA devices only (got %s); there is no CPU path" % device)
-        if dtype not in _DTYPES:
-            raise _lib.TdqError("unsupported state dtype %s (float32 and float64 are implemented)" % dtype)
+        self.dt_code, self.rt_code = state_codes(dtype)
         self.lib = _lib.load()
         self.fn = fn
         self.n = int(n)
         self.dtype = dtype
+        self.rdtype = dtype.to_real()   # dtype of time, step size and ratio (the component dtype of a complex state)
         self.device = device
-        self.dt_code = _DTYPES[dtype]
         self.tab = _lib.tableau(method)
         self.S = self.tab.n_stages
         self.fsal = bool(self.tab.fsal)
@@ -222,9 +231,9 @@ class AdaptiveEngine:
         self.rtol_vec = rtol_vec
         self.atol_vec = atol_vec
         vtol = rtol_vec is not None
-        self.ratio_f64 = vtol or dtype == torch.float64
+        self.ratio_f64 = vtol or self.rdtype == torch.float64
         self.opt = _lib.Options(
-            dtype=self.dt_code, ratio_f64=1 if vtol else 0,
+            dtype=self.rt_code, ratio_f64=1 if vtol else 0,
             rtol=float(rtol) if not vtol else 0.0, atol=float(atol) if not vtol else 0.0,
             min_step=float(min_step), max_step=float(max_step), safety=float(safety),
             ifactor=float(ifactor), dfactor=float(dfactor), t_sign=float(t_sign),
@@ -234,9 +243,9 @@ class AdaptiveEngine:
         kw = dict(dtype=dtype, device=device)
         self.ctrl = torch.zeros(self.lib.tdq_ctrl_size(), dtype=torch.uint8, device=device)
         o = self.lib.tdq_ctrl_tstage_offset()
-        self.tstage = self.ctrl[o:o + 8 * _lib.TDQ_MAX_K].view(dtype)
+        self.tstage = self.ctrl[o:o + 8 * _lib.TDQ_MAX_K].view(self.rdtype)
         o = self.lib.tdq_ctrl_taux_offset()
-        self.taux = self.ctrl[o:o + 32].view(dtype)
+        self.taux = self.ctrl[o:o + 32].view(self.rdtype)
         self.ybuf = [torch.zeros(self.n, **kw) for _ in range(2)]      # pointer table: accepted state ...
         self.kbuf = [torch.zeros(self.n, **kw) for _ in range(2)]      # ... and its derivative f0 = k_0
         self.opt.ybuf[0], self.opt.ybuf[1] = self.ybuf[0].data_ptr(), self.ybuf[1].data_ptr()
@@ -258,8 +267,9 @@ class AdaptiveEngine:
         self.qbuf = None
         self.ratio_buf = None
         if norm_fn is not None:
-            self.qbuf = torch.zeros(self.n, dtype=torch.float64 if vtol else dtype, device=device)
-            self.ratio_buf = torch.zeros((), dtype=torch.float64 if self.ratio_f64 else dtype, device=device)
+            qdt = dtype if not vtol else (torch.complex128 if dtype.is_complex else torch.float64)
+            self.qbuf = torch.zeros(self.n, dtype=qdt, device=device)
+            self.ratio_buf = torch.zeros((), dtype=torch.float64 if self.ratio_f64 else self.rdtype, device=device)
         self._own_ptrs = None
         self.mbox_host = C.POINTER(_lib.Mailbox)()
         mdev = C.c_void_p()
@@ -488,7 +498,7 @@ class AdaptiveEngine:
             ratio_ptr = self.ratio_buf.data_ptr()
         elif self.exchange is None:
             self._reduce(self.norm_out)
-        self._launch(lib.tdq_controller(ctrl, dc, self.norm_out.data_ptr(), self.seg_counts.data_ptr(), self.n_seg,
+        self._launch(lib.tdq_controller(ctrl, self.rt_code, self.norm_out.data_ptr(), self.seg_counts.data_ptr(), self.n_seg,
                                       ratio_ptr, st))
         return k, kp, keep
 
@@ -632,18 +642,18 @@ class AdaptiveEngine:
                 self._initial_step_custom_norm()
             else:
                 self._sumsq(self.kbuf[0], None, self.dsum[1])
-                self._launch(lib.tdq_initial_step_h0(ctrl, dc, self.dsum[0].data_ptr(), self.dsum[1].data_ptr(),
+                self._launch(lib.tdq_initial_step_h0(ctrl, self.rt_code, self.dsum[0].data_ptr(), self.dsum[1].data_ptr(),
                                                    self.seg_counts.data_ptr(), self.n_seg, st))
                 self._launch(lib.tdq_initial_step_probe(ctrl, dc, self.ytmp.data_ptr(), None, None, self.n, st))
                 f1 = self._eval(self.taux[1], self.ytmp, 1)
                 self._sumsq(f1, self.kbuf[0], self.dsum[2])
                 del f1
-                self._launch(lib.tdq_initial_step_finish(ctrl, dc, self.dsum[2].data_ptr(),
+                self._launch(lib.tdq_initial_step_finish(ctrl, self.rt_code, self.dsum[2].data_ptr(),
                                                        self.seg_counts.data_ptr(), self.n_seg, st))
         else:
             self._launch(lib.tdq_set_first_step(ctrl, float(self.first_step), st))
         bad_ptr = self.dsum[0].data_ptr() + 8 * self.n_seg if n_out > 1 else None
-        self._launch(lib.tdq_prepare_attempt(ctrl, dc, bad_ptr, st))
+        self._launch(lib.tdq_prepare_attempt(ctrl, self.rt_code, bad_ptr, st))
         return n_out
 
     # ---- lock step: the reference's exact call sequence --------------------------------------
@@ -898,7 +908,7 @@ class AdaptiveEngine:
 
     def _initial_step_custom_norm(self):
         """misc.py:36-77 with a user norm callable: torch ops + one host read (compatibility path)."""
-        T = self.dtype
+        T = self.rdtype
         y0, f0 = self.ybuf[0], self.kbuf[0] * self.opt.t_sign
         if self.rtol_vec is not None:
             scale = self.atol_vec + torch.abs(y0) * self.rtol_vec

@@ -8,7 +8,7 @@ grid interval, indexed by a device step counter."""
 import torch
 
 from . import _lib
-from ._engine import _DTYPES, _RetryWithCopies, _stream, pack_pieces, solver_stream
+from ._engine import _RetryWithCopies, _stream, pack_pieces, solver_stream, state_codes
 
 _ONE_THIRD = 1 / 3      # rk_common.py:94-96
 _TWO_THIRDS = 2 / 3
@@ -40,11 +40,9 @@ class FixedGridEngine:
         self.method = method
         if device.type != "cuda":
             raise _lib.TdqError("torchdiffeq_b200 runs on CUDA devices only (got %s); there is no CPU path" % device)
-        if dtype not in _DTYPES:
-            raise _lib.TdqError("unsupported state dtype %s (float32 and float64 are implemented)" % dtype)
+        self.dc = state_codes(dtype)[0]
         self.lib = _lib.load()
         self.fn, self.n, self.dtype, self.device = fn, int(n), dtype, device
-        self.dc = _DTYPES[dtype]
         self.t_sign = float(t_sign)
         self.perturb = bool(perturb)
         self.callbacks = callbacks or {}
@@ -59,10 +57,15 @@ class FixedGridEngine:
         self.nfe = 0
         self.launches = 0
 
+    @property
+    def rdtype(self):
+        """dtype of func's time argument, step sizes and interpolation weights: the component dtype of the state."""
+        return self.dtype.to_real()
+
     # ---- tables ---------------------------------------------------------------------------
     def _tabulate(self, grid, t):
         """grid, t: ascending CPU tensors of t's dtype.  Returns per-step and per-output tables."""
-        T = self.dtype
+        T = self.rdtype
         if grid.dtype != t.dtype:                  # a grid_constructor may return another float dtype: compare in
             common = torch.promote_types(grid.dtype, t.dtype)      # the promoted one, like the reference's mixed ops
             t = t.to(common)
@@ -246,12 +249,12 @@ class FixedGridEngine:
             self.cubic_dev, self.t1_dev = self._cubic.to(dev), self._t1_T.to(dev)
             self.rec_begin = torch.zeros_like(self.rec_begin)
         self.mode = mode.to(dev)
-        self.slope = slope.to(dev) if slope.numel() else torch.zeros(1, dtype=T, device=dev)
+        self.slope = slope.to(dev) if slope.numel() else torch.zeros(1, dtype=self.rdtype, device=dev)
         if self.out_idx.numel() == 0:
             self.out_idx = torch.zeros(1, dtype=torch.int32, device=dev)
             self.mode = torch.zeros(1, dtype=torch.int32, device=dev)
         self.step_dev = torch.zeros(2, dtype=torch.int64, device=dev)     # [0] step counter, [1] ticket of the emit kernel
-        self.tcur = self.ts_all[0].clone() if n_steps > 0 else torch.zeros(4, dtype=T, device=dev)
+        self.tcur = self.ts_all[0].clone() if n_steps > 0 else torch.zeros(4, dtype=self.rdtype, device=dev)
         kw = dict(dtype=T, device=dev)
         self.solution = torch.empty(t_cpu.numel(), self.n, **kw)
         self.solution[0].copy_(y0_flat)
@@ -324,7 +327,7 @@ class FixedGridEngine:
         import math
         dev, T = self.device, self.dtype
         kw = dict(dtype=T, device=dev)
-        t0c = torch.as_tensor(t0).detach().to("cpu").to(T).reshape(())              # t0.type_as(y0.abs())
+        t0c = torch.as_tensor(t0).detach().to("cpu").to(self.rdtype).reshape(())    # t0.type_as(y0.abs())
         dt = step_size.detach().to("cpu") if torch.is_tensor(step_size) else step_size
         self.solution = torch.empty(1, self.n, **kw)                                # nothing is emitted
         self.y0w = y0_flat.detach().clone()
@@ -332,7 +335,7 @@ class FixedGridEngine:
         self._own = {x.untyped_storage().data_ptr() for x in (self.y0w, self.ytmp, self.y1, self.solution)}
         z32 = torch.zeros(2, dtype=torch.int32, device=dev)
         self.rec_begin, self.out_idx, self.mode = z32, z32, z32
-        self.slope = torch.zeros(1, **kw)
+        self.slope = torch.zeros(1, dtype=self.rdtype, device=dev)
         self.n_steps = 1
         sign0 = torch.sign(event_fn(t0c.to(dev), self.y0w))
         itr = 0
@@ -352,7 +355,7 @@ class FixedGridEngine:
         y0, y1 = self.y0w, self.y1
         if self.interp == "cubic":
             f0 = keep[0] * self.t_sign
-            f1 = self._call_fn((t1c.to(T) * self.t_sign).to(dev), self.y1, None) * self.t_sign
+            f1 = self._call_fn((t1c.to(self.rdtype) * self.t_sign).to(dev), self.y1, None) * self.t_sign
 
             def interp_fn(t):                                                      # solvers.py:166-173
                 h = (t - t0c) / (t1c - t0c)
@@ -393,7 +396,7 @@ class FixedGridEngine:
     def _one_step_tables(self, t0c, dt, t1c):
         """Func times and dt of ONE step taken with an explicit dt (solvers.py:143-145 calls _step_func with
         dt = step_size, not t1 - t0), evaluated like the reference's 0-dim expressions."""
-        T, dev, m = self.dtype, self.device, self.method
+        T, dev, m = self.rdtype, self.device, self.method
         z = torch.zeros((), dtype=T)
         if m == "rk4":
             cols, prev_col = [t0c, t0c + dt * _ONE_THIRD, t0c + dt * _TWO_THIRDS, t1c], 3

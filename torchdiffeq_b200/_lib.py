@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libtdq.so")
 TDQ_MAX_STAGES = 16
 TDQ_MAX_K = TDQ_MAX_STAGES + 1
 TDQ_MAX_SEGS = 64
-TDQ_F32, TDQ_F64 = 0, 1
+TDQ_F32, TDQ_F64, TDQ_C64, TDQ_C128 = 0, 1, 2, 3     # complex: interleaved (re, im) pairs, n counts complex elements
 RUN_OK, RUN_DT_UNDERFLOW, RUN_NONFINITE, RUN_MAX_STEPS, RUN_EXCHANGE_TIMEOUT = 0, 1, 2, 3, 4
 TDQ_MAX_RANKS = 16
 ABI_VERSION = 2

@@ -240,7 +240,7 @@ class _BackwardSolver:
         time_vjps = torch.empty(len(t), dtype=t.dtype, device=t.device) if self.t_requires_grad else None
         for i in range(len(t) - 1, 0, -1):                            # adjoint.py:124-141
             if self.t_requires_grad:
-                fe = self.base_fn(t[i].to(T), y[i])
+                fe = self.base_fn(t[i].to(T.to_real()), y[i])
                 if isinstance(fe, tuple):
                     fe = self.fwd_layout.flatten([f_.detach() for f_ in fe])
                 dLd_cur_t = fe.reshape(-1).dot(grad_sol[i].reshape(-1))
@@ -402,6 +402,11 @@ def odeint_adjoint(func, y0, t, *, rtol=1e-7, atol=1e-9, method=None, options=No
                           "excluded from the adjoint pass, and will not appear as a tensor in the adjoint norm.")
 
     p = normalise(func, y0, t, rtol, atol, method, options, event_fn)
+    if p.dtype.is_complex and not all(q.is_complex() for q in adjoint_params):
+        # the augmented state [vjp_t | y | adj_y | theta...] is one complex vector, so a real parameter would receive a
+        # complex gradient (the reference fails inside autograd here)
+        raise TypeError("odeint_adjoint with a complex state needs complex adjoint parameters; got real ones: %s"
+                        % [tuple(q.shape) for q in adjoint_params if not q.is_complex()])
     if adjoint_method is None:
         adjoint_method = 'dopri5'
     if adjoint_method not in ADAPTIVE_METHODS + FIXED_METHODS:

@@ -94,6 +94,7 @@ template <> struct Ar<float> {
         return (a != a || b != b) ? CUDART_NAN_F : fmaxf(a, b);
     }
     static __device__ __forceinline__ bool finite(float a) { return isfinite(a); }
+    static __device__ __forceinline__ float cabs(float re, float im) { return hypotf(re, im); }   // torch's complex abs
 };
 template <> struct Ar<double> {
     static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
@@ -105,6 +106,7 @@ template <> struct Ar<double> {
         return (a != a || b != b) ? CUDART_NAN : fmax(a, b);
     }
     static __device__ __forceinline__ bool finite(double a) { return isfinite(a); }
+    static __device__ __forceinline__ double cabs(double re, double im) { return hypot(re, im); }
 };
 
 // ------------------------------------------------------------------------------------------------

@@ -245,6 +245,7 @@ int tdq_rk4_stage(int32_t dtype, int32_t which, void *y_out, const void *y0, con
                   const void *k3, const void *k4, const void *dt_dev, const int64_t *step_dev, size_t n,
                   void *stream) {
     TDQ_REQUIRE(y_out && y0 && dt_dev, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TDQ_REQUIRE(which >= 1 && which <= 9, "which must be 1..9");
     const bool nA = which != 8, nB = which == 2 || which == 3 || which == 4 || which == 7 || which == 8,
                nC = which == 3 || which == 4 || which == 9, nD = which == 4;
@@ -277,6 +278,7 @@ int tdq_fixed_emit(int32_t dtype, void *y0, const void *y1, void *solution, cons
     TDQ_REQUIRE(y0 && y1 && solution && rec_begin_dev && out_idx_dev && mode_dev && slope_dev && step_dev &&
                     tstage_all_dev && tstage_cur_dev,
                 "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     cudaStream_t st = (cudaStream_t)stream;
     size_t blocks = (n + kThreads - 1) / kThreads;
     if (blocks == 0) blocks = 1;
@@ -299,6 +301,7 @@ int tdq_fixed_final_emit(int32_t dtype, int32_t which, void *y0, const void *k1,
     TDQ_REQUIRE(which == 4 || which == 5 || which == 7 || which == 9, "which must be a final expression (4, 5, 7, 9)");
     TDQ_REQUIRE(k1 && (which == 5 || which == 9 || k2) && (which != 4 && which != 9 || k3) && (which != 4 || k4),
                 "missing stage slot");
+    TDQ_REAL_VIEW(dtype, n);
     cudaStream_t st = (cudaStream_t)stream;
     size_t blocks = (n + kThreads - 1) / kThreads;
     if (blocks == 0) blocks = 1;
@@ -319,6 +322,7 @@ int tdq_fixed_final_emit(int32_t dtype, int32_t which, void *y0, const void *k1,
 int tdq_lincomb(int32_t dtype, void *out, const void *base, const void *const *x, const double *coefs, int32_t n_terms,
                 size_t n, void *stream) {
     TDQ_REQUIRE(out && x && coefs, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TDQ_REQUIRE(n_terms >= 1 && n_terms <= TDQ_MAX_K, "n_terms out of range");
     LinArgs a;
     memset(&a, 0, sizeof(a));
@@ -340,6 +344,7 @@ int tdq_fixed_emit_cubic(int32_t dtype, const void *y0, const void *y1, const vo
                          const int32_t *out_idx_dev, const void *coef_dev, int32_t rec_lo, int32_t rec_hi, size_t n,
                          void *stream) {
     TDQ_REQUIRE(y0 && y1 && f0 && f1 && solution && out_idx_dev && coef_dev, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TDQ_REQUIRE(rec_lo >= 0 && rec_hi >= rec_lo, "bad record range");
     if (n == 0 || rec_hi == rec_lo) return TDQ_OK;
     size_t blocks = (n + kThreads - 1) / kThreads;
@@ -355,16 +360,18 @@ int tdq_pack_segments(int32_t dtype, void *dst, const void *const *src, const in
                       const double *scales, int32_t n_src, void *stream) {
     TDQ_REQUIRE(dst && src && offsets && lens && scales, "null argument");
     TDQ_REQUIRE(n_src >= 1 && n_src <= TDQ_MAX_SEGS, "n_src out of range");
+    size_t w = 1;                                   // components per element
+    TDQ_REAL_VIEW(dtype, w);
     PackArgs a;
     memset(&a, 0, sizeof(a));
     int64_t max_len = 0;
     for (int i = 0; i < n_src; ++i) {
-        a.src[i] = src[i];
-        a.off[i] = offsets[i];
-        a.len[i] = lens[i];
-        a.scale[i] = scales[i];
         TDQ_REQUIRE(lens[i] >= 0 && offsets[i] >= 0, "negative segment");
-        if (lens[i] > max_len) max_len = lens[i];
+        a.src[i] = src[i];
+        a.off[i] = offsets[i] * (int64_t)w;
+        a.len[i] = lens[i] * (int64_t)w;
+        a.scale[i] = scales[i];
+        if (a.len[i] > max_len) max_len = a.len[i];
     }
     if (max_len == 0) return TDQ_OK;
     size_t bx = (size_t)((max_len + kThreads * 4 - 1) / (kThreads * 4));

@@ -200,6 +200,7 @@ extern "C" {
 int tdq_initial_step_probe(void *ctrl_dev, int32_t dtype, void *y_probe, const void *y0, const void *f0, size_t n,
                            void *stream) {
     TDQ_REQUIRE(ctrl_dev && y_probe, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     if (n == 0) return TDQ_OK;
     size_t blocks = (n + kThreads - 1) / kThreads;
     if (blocks > (size_t)tdq_sm_count() * 16) blocks = (size_t)tdq_sm_count() * 16;
@@ -212,6 +213,7 @@ int tdq_initial_step_probe(void *ctrl_dev, int32_t dtype, void *y_probe, const v
 int tdq_interp_fit_eval(void *ctrl_dev, const tdq_tableau *tab, int32_t dtype, const void *y1, const void *const *k,
                         void *const *coeff, void *solution, size_t n, void *stream) {
     TDQ_REQUIRE(ctrl_dev && tab && y1 && k && solution, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TdqHostShape hs;
     tdq_shape_from_tableau(tab, &hs);
     const int S = hs.n_stages;
@@ -244,6 +246,7 @@ int tdq_interp_fit_eval(void *ctrl_dev, const tdq_tableau *tab, int32_t dtype, c
 
 int tdq_poly_eval(int32_t dtype, const void *const *coeff, double x, void *out, size_t n, void *stream) {
     TDQ_REQUIRE(coeff && out, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     for (int i = 0; i < 5; ++i) TDQ_REQUIRE(coeff[i] != nullptr, "five coefficient buffers are required");
     if (n == 0) return TDQ_OK;
     size_t blocks = (n + kThreads - 1) / kThreads;
@@ -258,6 +261,7 @@ int tdq_poly_eval(int32_t dtype, const void *const *coeff, double x, void *out, 
 int tdq_interp_eval_at(void *ctrl_dev, int32_t dtype, const void *const *coeff, const double *t_dev, void *out,
                        size_t n, void *stream) {
     TDQ_REQUIRE(ctrl_dev && coeff && out && t_dev, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     for (int i = 0; i < 5; ++i) TDQ_REQUIRE(coeff[i] != nullptr, "five coefficient buffers are required");
     if (n == 0) return TDQ_OK;
     size_t blocks = (n + kThreads - 1) / kThreads;

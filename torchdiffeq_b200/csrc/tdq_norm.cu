@@ -9,6 +9,11 @@
 //   MODE 1  out[s] = sum (x / scale)^2,         scale = atol + |y0| * rtol          misc.py:55-58
 //   MODE 2  out[s] = sum ((x - x2) / scale)^2                                       misc.py:69
 //
+// Complex states (CPX): T is the component dtype and an element is an interleaved (re, im) pair.  |.| is the modulus
+// (hypot, what torch's complex abs computes), tol and scale stay real, x/tol is x * fl(1/tol) componentwise (torch's
+// complex-by-real division), and an element adds |x/tol|^2 = fl(fl(hypot(q))^2) once (.abs().pow(2)); it is non-finite
+// when either part is.  Indices, segments and chunk lengths count elements; a chunk holds at most kChunk components.
+//
 // Work decomposition.  Single segment covering [0, n): a persistent grid of at most kMaxGrid blocks,
 // thread-local float64 accumulation over a fixed block-strided assignment, one partial per block.
 // Several segments (tuple states, the adjoint's augmented state, any number of them): a CHUNK TABLE in
@@ -29,6 +34,9 @@ constexpr int kMaxGrid = 148 * 4;       // persistent grid of the single-segment
 template <typename T, bool VTOL> struct TolT { using type = T; };
 template <typename T> struct TolT<T, true> { using type = double; };
 
+// components per element
+template <bool CPX> constexpr int kWidth = CPX ? 2 : 1;
+
 struct NormArgs {
     const void *x;          // MODE 0: err_pre          MODE 1/2: x
     const void *x2;         // MODE 0: k_S              MODE 2: x2
@@ -38,13 +46,13 @@ struct NormArgs {
     const int64_t *table;   // chunk table (MULTI) or NULL
     double *partials;       // [0..1]: ticket word; then sums[P], then bad[P]
     double *out;            // [n_seg + 1]
-    void *q_out;            // WRITEQ: err/tol per element
-    size_t n;
+    void *q_out;            // WRITEQ: err/tol per element (a pair per complex element)
+    size_t n;               // elements
     int n_parts;            // P: blocks (single) or chunks (multi)
     int n_seg;
 };
 
-template <typename T, int MODE, bool VECTOR, bool VTOL, bool MULTI, bool WRITEQ>
+template <typename T, bool CPX, int MODE, bool VECTOR, bool VTOL, bool MULTI, bool WRITEQ>
 __global__ void __launch_bounds__(kThreads)
 k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
     if (c->halt) return;
@@ -52,6 +60,8 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
     using Q = typename TolT<T, VTOL>::type;     // dtype of tol and of err/tol (float64 with vector tolerances)
     using V = Vec<T>;
     constexpr int VN = VECTOR ? V::N : 1;
+    constexpr int EW = kWidth<CPX>;             // components per element
+    constexpr int VE = V::N / EW;               // elements per 16-byte vector
     __shared__ double red[kThreads / 32];
     __shared__ bool is_last;
 
@@ -96,18 +106,78 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
         const Q q2 = Ar<Q>::mul(q, q);                 // .abs().pow(2)
         acc += (double)q2;
     };
+    // one complex element: v0 = y0[i], v1 = y1[i], xa = x[i], xb = x2[i] as (re, im) pairs
+    auto celement = [&](size_t i, const T *v0, const T *v1, const T *xa, const T *xb, bool in_seg) {
+        if (MODE == 0 && !(A::finite(v1[0]) && A::finite(v1[1]))) bad += 1.0;
+        if (MODE == 1 && !(A::finite(v0[0]) && A::finite(v0[1]))) bad += 1.0;
+        if (!in_seg) return;
+        T num[2];
+#pragma unroll
+        for (int p = 0; p < 2; ++p) {
+            if (MODE == 0) num[p] = ek ? A::add(xa[p], A::mul(xb[p], ecS)) : xa[p];
+            else num[p] = (MODE == 2) ? A::sub(xa[p], xb[p]) : xa[p];
+        }
+        const T m0 = A::cabs(v0[0], v0[1]);
+        Q q[2];
+        if (VTOL) {
+            const double rt = a.rtol_v[i], at = a.atol_v[i];
+            double tol;
+            if (MODE == 0) tol = at + rt * (double)A::max_nan(m0, A::cabs(v1[0], v1[1]));
+            else tol = at + (double)m0 * rt;
+            const double r = 1.0 / tol;
+            q[0] = (Q)((double)num[0] * r);
+            q[1] = (Q)((double)num[1] * r);
+        } else {
+            T tol;
+            if (MODE == 0) tol = A::add(atolT, A::mul(rtolT, A::max_nan(m0, A::cabs(v1[0], v1[1]))));
+            else tol = A::add(atolT, A::mul(m0, rtolT));
+            const T r = A::div((T)1, tol);
+            q[0] = (Q)A::mul(num[0], r);
+            q[1] = (Q)A::mul(num[1], r);
+        }
+        if (WRITEQ) {
+            reinterpret_cast<Q *>(a.q_out)[2 * i] = q[0];
+            reinterpret_cast<Q *>(a.q_out)[2 * i + 1] = q[1];
+        }
+        const Q m = Ar<Q>::cabs(q[0], q[1]);
+        acc += (double)Ar<Q>::mul(m, m);               // .abs().pow(2)
+    };
     auto scalar_at = [&](size_t i, bool in_seg) {
-        const T v1 = (MODE == 0) ? y1[i] : (T)0;
-        const T xb = (MODE != 1) ? x2[i] : (T)0;
-        element(i, y0[i], v1, x[i], xb, in_seg);
-        if (MODE == 0 && ycand) { ycand[i] = v1; kcand[i] = xb; }
+        if constexpr (CPX) {
+            const size_t j = 2 * i;
+            const T v0[2] = {y0[j], y0[j + 1]};
+            const T xa[2] = {x[j], x[j + 1]};
+            const T v1[2] = {(MODE == 0) ? y1[j] : (T)0, (MODE == 0) ? y1[j + 1] : (T)0};
+            const T xb[2] = {(MODE != 1) ? x2[j] : (T)0, (MODE != 1) ? x2[j + 1] : (T)0};
+            celement(i, v0, v1, xa, xb, in_seg);
+            if (MODE == 0 && ycand) {
+                ycand[j] = v1[0]; ycand[j + 1] = v1[1];
+                kcand[j] = xb[0]; kcand[j + 1] = xb[1];
+            }
+        } else {
+            const T v1 = (MODE == 0) ? y1[i] : (T)0;
+            const T xb = (MODE != 1) ? x2[i] : (T)0;
+            element(i, y0[i], v1, x[i], xb, in_seg);
+            if (MODE == 0 && ycand) { ycand[i] = v1; kcand[i] = xb; }
+        }
+    };
+    // the VE elements of one 16-byte vector, the first of which is element i
+    auto vector_at = [&](size_t i, const V &a0, const V &a1, const V &xa, const V &xb, bool in_seg) {
+#pragma unroll
+        for (int e = 0; e < VE; ++e) {
+            if constexpr (CPX)
+                celement(i + e, &a0.v[2 * e], &a1.v[2 * e], &xa.v[2 * e], &xb.v[2 * e], in_seg);
+            else
+                element(i + e, a0.v[e], (MODE == 0) ? a1.v[e] : (T)0, xa.v[e], (MODE != 1) ? xb.v[e] : (T)0,
+                        in_seg);
+        }
     };
 
     if (!MULTI) {
         // ---- one segment = [0, n): persistent blocks, fixed block-strided assignment -------------------
         constexpr int U = 2;
         if (VECTOR) {
-            const size_t nvec = a.n / V::N;
+            const size_t nvec = a.n / VE;
             const size_t stride = (size_t)gridDim.x * (kThreads * U);
             for (size_t base = (size_t)blockIdx.x * (kThreads * U) + threadIdx.x; base < nvec; base += stride) {
                 V a0[U], a1[U], xa[U], xb[U];
@@ -127,10 +197,7 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
                     const size_t v = base + (size_t)u * kThreads;
                     if (v < nvec) {
                         const size_t i0 = v * V::N;
-#pragma unroll
-                        for (int e = 0; e < V::N; ++e)
-                            element(i0 + e, a0[u].v[e], (MODE == 0) ? a1[u].v[e] : (T)0, xa[u].v[e],
-                                    (MODE != 1) ? xb[u].v[e] : (T)0, true);
+                        vector_at(v * VE, a0[u], a1[u], xa[u], xb[u], true);
                         if (MODE == 0 && ycand) {
                             st_vec<T>(ycand + i0, a1[u]);
                             st_vec<T>(kcand + i0, xb[u]);
@@ -139,7 +206,7 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
                 }
             }
             if (blockIdx.x == 0) {
-                const size_t i = nvec * V::N + threadIdx.x;
+                const size_t i = nvec * VE + threadIdx.x;
                 if (i < a.n) scalar_at(i, true);
             }
         } else {
@@ -158,7 +225,8 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
         const int n_seg = (int)tb[0], n_chunks = (int)tb[1];
         const int64_t *chunk_start = tb + 4 + 2 * (int64_t)n_seg;
         const int64_t *chunk_meta = chunk_start + n_chunks;
-        constexpr int U = kChunk / (kThreads * VN);
+        // slots per thread: a chunk holds at most kChunk components, i.e. kChunk / V::N vectors or kChunk / EW elements
+        constexpr int U = kChunk / (kThreads * (VECTOR ? VN : EW));
         for (int ch = blockIdx.x; ch < n_chunks; ch += gridDim.x) {
             const int64_t start = chunk_start[ch], meta = chunk_meta[ch];
             const int len = (int)(meta & 0xffffffffll);
@@ -167,13 +235,13 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
             bad = 0.0;
             if (in_seg || MODE == 0) {
                 if (VECTOR) {
-                    const int nvec = len / V::N;
+                    const int nvec = len / VE;
                     V a0[U], a1[U], xa[U], xb[U];
 #pragma unroll
                     for (int u = 0; u < U; ++u) {
                         const int v = threadIdx.x + u * kThreads;
                         if (v < nvec) {
-                            const size_t i0 = (size_t)start + (size_t)v * V::N;
+                            const size_t i0 = ((size_t)start + (size_t)v * VE) * EW;
                             a0[u] = ld_stream<T>(y0 + i0);
                             xa[u] = ld_stream<T>(x + i0);
                             if (MODE == 0) a1[u] = ld_stream<T>(y1 + i0);
@@ -184,18 +252,15 @@ k_norm(const TdqCtrl *__restrict__ c, NormArgs a) {
                     for (int u = 0; u < U; ++u) {
                         const int v = threadIdx.x + u * kThreads;
                         if (v < nvec) {
-                            const size_t i0 = (size_t)start + (size_t)v * V::N;
-#pragma unroll
-                            for (int e = 0; e < V::N; ++e)
-                                element(i0 + e, a0[u].v[e], (MODE == 0) ? a1[u].v[e] : (T)0, xa[u].v[e],
-                                        (MODE != 1) ? xb[u].v[e] : (T)0, in_seg);
+                            const size_t i0 = ((size_t)start + (size_t)v * VE) * EW;
+                            vector_at((size_t)start + (size_t)v * VE, a0[u], a1[u], xa[u], xb[u], in_seg);
                             if (MODE == 0 && ycand) {
                                 st_vec<T>(ycand + i0, a1[u]);
                                 st_vec<T>(kcand + i0, xb[u]);
                             }
                         }
                     }
-                    const int i = nvec * V::N + threadIdx.x;
+                    const int i = nvec * VE + threadIdx.x;
                     if (i < len) scalar_at((size_t)start + i, in_seg);
                 } else {
 #pragma unroll
@@ -279,7 +344,7 @@ k_commit(const TdqCtrl *__restrict__ c, const T *__restrict__ y1, const T *__res
     }
 }
 
-template <typename T, int MODE>
+template <typename T, bool CPX, int MODE>
 int launch_norm(const TdqCtrl *c, NormArgs &a, bool vec, cudaStream_t st) {
     const bool vtol = a.rtol_v != nullptr;
     const bool multi = a.table != nullptr;
@@ -293,7 +358,7 @@ int launch_norm(const TdqCtrl *c, NormArgs &a, bool vec, cudaStream_t st) {
         grid = (unsigned)a.n_parts;
     }
     if (grid == 0) grid = 1;
-#define TDQ_L(V_, VT_, M_, WQ_) k_norm<T, MODE, V_, VT_, M_, WQ_><<<grid, kThreads, 0, st>>>(c, a)
+#define TDQ_L(V_, VT_, M_, WQ_) k_norm<T, CPX, MODE, V_, VT_, M_, WQ_><<<grid, kThreads, 0, st>>>(c, a)
 #define TDQ_L3(V_, VT_, M_) do { if (wq && MODE == 0) TDQ_L(V_, VT_, M_, (MODE == 0)); else TDQ_L(V_, VT_, M_, false); } while (0)
 #define TDQ_L2(V_, VT_) do { if (multi) TDQ_L3(V_, VT_, true); else TDQ_L3(V_, VT_, false); } while (0)
     if (vec) { if (vtol) TDQ_L2(true, true); else TDQ_L2(true, false); }
@@ -303,6 +368,21 @@ int launch_norm(const TdqCtrl *c, NormArgs &a, bool vec, cudaStream_t st) {
 #undef TDQ_L
     return 0;
 }
+
+// k_norm for a state dtype code; -1 for a code that is not one
+template <int MODE>
+int dispatch_norm(int32_t dtype, const TdqCtrl *c, NormArgs &a, bool vec, cudaStream_t st) {
+    switch (dtype) {
+        case TDQ_F32: return launch_norm<float, false, MODE>(c, a, vec, st);
+        case TDQ_F64: return launch_norm<double, false, MODE>(c, a, vec, st);
+        case TDQ_C64: return launch_norm<float, true, MODE>(c, a, vec, st);
+        case TDQ_C128: return launch_norm<double, true, MODE>(c, a, vec, st);
+        default: return -1;
+    }
+}
+
+// elements per 16-byte vector of a state dtype (4 float32, 2 float64 or complex64, 1 complex128)
+inline int vec_elems(int32_t dtype) { return 16 / (tdq_dtype_width(dtype) * (tdq_real_code(dtype) == TDQ_F32 ? 4 : 8)); }
 
 // number of partials (= blocks) of the single-segment path for n elements
 inline int single_parts(size_t n, bool vec, int vn) {
@@ -332,11 +412,12 @@ int64_t tdq_norm_table_fill(const int64_t *seg_offsets, const int64_t *seg_lens,
     // Layout: [n_seg, n_chunks, kChunk, aligned] seg_first[n_seg] seg_nchunks[n_seg] chunk_start[n_chunks]
     // chunk_meta[n_chunks] (len | (segment+1) << 32; 0 = gap).  Gaps are cut so that every chunk of at least
     // one 16-byte vector starts on a 16-byte boundary; `aligned` says whether every SEGMENT does too.
-    if (!seg_offsets || !seg_lens || n_seg < 1 || n < 0 || (dtype != TDQ_F32 && dtype != TDQ_F64)) {
+    if (!seg_offsets || !seg_lens || n_seg < 1 || n < 0 || tdq_dtype_width(dtype) == 0) {
         tdq_set_error("tdq_norm_table_fill: bad argument");
         return -1;
     }
-    const int64_t vn = dtype == TDQ_F32 ? 4 : 2;
+    const int64_t vn = vec_elems(dtype);
+    const int64_t kChunk = ::kChunk / tdq_dtype_width(dtype);   // elements per chunk: at most kChunk components
     int64_t ch = 0;
     int64_t *seg_first = nullptr, *seg_nch = nullptr, *chunk_start = nullptr, *chunk_meta = nullptr;
     bool write = false;
@@ -391,7 +472,7 @@ int64_t tdq_norm_table_fill(const int64_t *seg_offsets, const int64_t *seg_lens,
 
 static int norm_common(NormArgs &a, const int64_t *table_dev, int64_t n_chunks, int32_t n_seg, int32_t dtype,
                        bool table_aligned, bool *vec) {
-    const int vn = dtype == TDQ_F32 ? 4 : 2;
+    const int vn = vec_elems(dtype);
     a.table = table_dev;
     a.n_seg = n_seg;
     if (table_dev) {
@@ -411,6 +492,7 @@ int tdq_error_norm_commit(void *ctrl_dev, int32_t dtype, const void *err_pre, co
                           double *out, void *err_over_tol_out, void *stream) {
     TDQ_REQUIRE(ctrl_dev && err_pre && k_last && y1 && partials && out, "null argument");
     TDQ_REQUIRE(n_seg >= 1, "n_seg out of range");
+    TDQ_REQUIRE(tdq_dtype_width(dtype) != 0, "unsupported dtype");
     TDQ_REQUIRE((rtol_vec == nullptr) == (atol_vec == nullptr), "rtol_vec and atol_vec go together");
     NormArgs a;
     memset(&a, 0, sizeof(a));
@@ -422,7 +504,7 @@ int tdq_error_norm_commit(void *ctrl_dev, int32_t dtype, const void *err_pre, co
     TDQ_REQUIRE(norm_common(a, table_dev, n_chunks, n_seg, dtype, table_aligned != 0, &vec) == 0,
                 "several segments need a chunk table (tdq_norm_table_fill)");
     if (n == 0) return TDQ_OK;
-    TDQ_DISPATCH_T(dtype, (launch_norm<T, 0>((const TdqCtrl *)ctrl_dev, a, vec, (cudaStream_t)stream)));
+    dispatch_norm<0>(dtype, (const TdqCtrl *)ctrl_dev, a, vec, (cudaStream_t)stream);
     TDQ_CHECK_CUDA(cudaGetLastError());
     return TDQ_OK;
 }
@@ -432,6 +514,7 @@ int tdq_scaled_sumsq(void *ctrl_dev, int32_t dtype, const void *x, const void *x
                      int32_t table_aligned, int32_t n_seg, size_t n, double *partials, double *out, void *stream) {
     TDQ_REQUIRE(ctrl_dev && x && partials && out, "null argument");
     TDQ_REQUIRE(n_seg >= 1, "n_seg out of range");
+    TDQ_REQUIRE(tdq_dtype_width(dtype) != 0, "unsupported dtype");
     TDQ_REQUIRE((rtol_vec == nullptr) == (atol_vec == nullptr), "rtol_vec and atol_vec go together");
     NormArgs a;
     memset(&a, 0, sizeof(a));
@@ -444,14 +527,15 @@ int tdq_scaled_sumsq(void *ctrl_dev, int32_t dtype, const void *x, const void *x
     if (n == 0) return TDQ_OK;
     const TdqCtrl *c = (const TdqCtrl *)ctrl_dev;
     cudaStream_t st = (cudaStream_t)stream;
-    if (x2) TDQ_DISPATCH_T(dtype, (launch_norm<T, 2>(c, a, vec, st)));
-    else TDQ_DISPATCH_T(dtype, (launch_norm<T, 1>(c, a, vec, st)));
+    if (x2) dispatch_norm<2>(dtype, c, a, vec, st);
+    else dispatch_norm<1>(dtype, c, a, vec, st);
     TDQ_CHECK_CUDA(cudaGetLastError());
     return TDQ_OK;
 }
 
 int tdq_commit_candidates(void *ctrl_dev, int32_t dtype, const void *y1, const void *k_last, size_t n, void *stream) {
     TDQ_REQUIRE(ctrl_dev && y1 && k_last, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     if (n == 0) return TDQ_OK;
     size_t blocks = (n + kThreads - 1) / kThreads;
     const size_t cap = (size_t)tdq_sm_count() * 8;

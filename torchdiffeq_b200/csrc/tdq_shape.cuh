@@ -26,3 +26,24 @@ int tdq_sm_count();                                                     // tdq_s
         else if ((dtype) == TDQ_F64) { using T = double; __VA_ARGS__; }    \
         else { tdq_set_error("unsupported dtype %d", (int)(dtype)); return TDQ_ERR_INVALID; } \
     } while (0)
+
+// Components per element of a state dtype: 1 (real), 2 (complex: interleaved re, im), 0 (not a dtype code).
+static inline int tdq_dtype_width(int32_t dtype) {
+    return (dtype == TDQ_F32 || dtype == TDQ_F64) ? 1 : (dtype == TDQ_C64 || dtype == TDQ_C128) ? 2 : 0;
+}
+// The component dtype of a state dtype (itself for real codes).
+static inline int32_t tdq_real_code(int32_t dtype) {
+    return dtype == TDQ_C64 ? TDQ_F32 : dtype == TDQ_C128 ? TDQ_F64 : dtype;
+}
+
+// The one place that knows what a complex state is to a launcher whose arithmetic only applies REAL coefficients
+// (stage combines, the probe, the interpolant, fixed-grid steps, Adams sums, the pack, copies): z * (c + 0i) is
+// (re * c, im * c) bit for bit, so such a launcher runs its real kernel on the 2n components of n complex elements.
+// Rewrites (dtype, n) to (component dtype, components); refuses unknown codes.
+#define TDQ_REAL_VIEW(dtype, n)                                                               \
+    do {                                                                                      \
+        const int w_ = tdq_dtype_width(dtype);                                                \
+        if (w_ == 0) { tdq_set_error("%s: unsupported dtype %d", __func__, (int)(dtype)); return TDQ_ERR_INVALID; } \
+        (n) *= w_;                                                                            \
+        (dtype) = tdq_real_code(dtype);                                                       \
+    } while (0)

@@ -321,6 +321,7 @@ extern "C" {
 int tdq_stage_combine(void *ctrl_dev, const tdq_tableau *tab, int32_t dtype, int32_t row, void *y_out,
                       const void *y0, const void *const *k, size_t n, void *stream) {
     TDQ_REQUIRE(ctrl_dev && tab && y_out && k, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TdqHostShape hs;
     tdq_shape_from_tableau(tab, &hs);
     TDQ_REQUIRE(row >= 0 && row <= hs.n_stages, "row out of range");
@@ -347,6 +348,7 @@ int tdq_stage_combine(void *ctrl_dev, const tdq_tableau *tab, int32_t dtype, int
 int tdq_stage_combine_final(void *ctrl_dev, const tdq_tableau *tab, int32_t dtype, void *y1_out, void *err_out,
                             const void *y0, const void *const *k, size_t n, void *stream) {
     TDQ_REQUIRE(ctrl_dev && tab && y1_out && err_out && k, "null argument");
+    TDQ_REAL_VIEW(dtype, n);
     TdqHostShape hs;
     tdq_shape_from_tableau(tab, &hs);
     const int S = hs.n_stages;

@@ -113,13 +113,21 @@ def normalise(func, y0, t, rtol, atol, method, options, event_fn, adjoint=False)
     p.is_tuple = not isinstance(y0, torch.Tensor)
     if p.is_tuple:
         assert isinstance(y0, tuple), 'y0 must be either a torch.Tensor or a tuple'   # misc.py:216
-        p.layout = Layout([y_.shape for y_ in y0], y0[0].dtype)
-        p.device = y0[0].device
         p.dtype = y0[0].dtype
+        if any(y_.dtype.is_complex for y_ in y0):
+            # the reference's torch.cat promotes a tuple with a complex piece: every piece integrates (and comes back)
+            # in the common complex dtype
+            for y_ in y0[1:]:
+                p.dtype = torch.promote_types(p.dtype, y_.dtype)
+        p.layout = Layout([y_.shape for y_ in y0], p.dtype)
+        p.device = y0[0].device
     else:
         p.layout = None
         p.device = y0.device
         p.dtype = y0.dtype
+    if torch.complex32 in ([y_.dtype for y_ in y0] if p.is_tuple else [p.dtype]):
+        raise _lib.TdqError("unsupported state dtype torch.complex32 (float32, float64, complex64 and complex128 are "
+                            "implemented)")
     options = {} if options is None else options.copy()                               # misc.py:226-229
     if method is None:
         method = 'dopri5'
@@ -130,6 +138,9 @@ def normalise(func, y0, t, rtol, atol, method, options, event_fn, adjoint=False)
         raise NotImplementedError('method "{}" is not part of the B200 hot path; implemented: {}'.format(
             method, ADAPTIVE_METHODS + FIXED_METHODS + tuple(ADAMS_METHODS)))
     p.method, p.options = method, options
+    if p.dtype.is_complex and options.get("process_group") is not None:
+        raise NotImplementedError("batch-sharded solves (options['process_group']) of a complex state are not "
+                                  "implemented")
     if p.device.type != "cuda":
         raise _lib.TdqError("torchdiffeq_b200 runs on CUDA devices only (got %s); there is no CPU path" % p.device)
     _lib.load()                                   # fail loudly, before any work, if libtdq.so is missing
@@ -654,6 +665,9 @@ def _odeint_backprop(p, func, y0, t, params, _stats):
     """Plain odeint under autograd: gradients of the discrete solve w.r.t. y0, t and every parameter func reaches
     (odeint.py:49-108 differentiated as the reference's recorded graph would be; see backprop.py)."""
     from .backprop import _BackpropFunction, adaptive_tableau
+    if p.dtype.is_complex:
+        raise NotImplementedError("gradients of the discrete solve of a complex state are not implemented; use "
+                                  "odeint_adjoint, or call odeint under torch.no_grad()")
     if p.is_tuple:
         y0_flat = p.layout.flatten(list(y0))          # differentiable w.r.t. every piece
     else:

@@ -249,6 +249,9 @@ def make_fixed(method, **defaults):
     return B200FixedSolver
 
 
+_STATE_DTYPES = (torch.float32, torch.float64, torch.complex64, torch.complex128)
+
+
 class _Dispatch:
     """What goes into SOLVERS[name]: callable like a solver class, routes CUDA states to libtdq and everything else
     to the class that was registered before."""
@@ -257,8 +260,7 @@ class _Dispatch:
         self.name, self.gpu_cls, self.cpu_cls = name, gpu_cls, cpu_cls
 
     def __call__(self, func, y0, **kwargs):
-        cls = self.gpu_cls if (torch.is_tensor(y0) and y0.is_cuda and y0.dtype in (torch.float32, torch.float64)) \
-            else self.cpu_cls
+        cls = self.gpu_cls if (torch.is_tensor(y0) and y0.is_cuda and y0.dtype in _STATE_DTYPES) else self.cpu_cls
         if cls is None:
             raise _lib.TdqError("no solver registered for %s on %s" % (self.name, y0.device))
         return cls(func=func, y0=y0, **kwargs)
